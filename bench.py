@@ -62,7 +62,37 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-vit-sweep", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed paths computed in their last step to DIR/<name>.npy (float32 / float64)")
     return ap.parse_args()
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Last-step outputs of the timed paths as DIR/<name>.npy: floats as float32, token ids as float64 (exact). Same
+    arguments -> same seeded inputs, so two builds can be compared output for output. Whole-array unless noted; a
+    larger output is a fixed, seeded sample (<= 64 MB in all)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        if torch.is_tensor(t):
+            t = t.detach()
+            a = (t.float() if t.is_floating_point() else t).cpu().numpy()
+        else:
+            a = np.asarray(t)
+        a = a.astype(np.float32 if a.dtype.kind == "f" else np.float64)
+        total += a.nbytes
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    assert total <= 64 << 20, total
+
+
+def seeded_sample(t: torch.Tensor, n: int, seed: int = 0) -> torch.Tensor:
+    """A fixed, seeded sample of n elements of t (all of t when it is not larger)."""
+    flat = t.reshape(-1)
+    if flat.numel() <= n:
+        return flat
+    idx = torch.randint(flat.numel(), (n,), generator=torch.Generator().manual_seed(seed)).sort().values
+    return flat[idx.to(flat.device)]
 
 
 # ---------------------------------------------------------------------------------- clocks
@@ -300,7 +330,7 @@ def run_ours(args):
             ev[2].record(stream)
         out = eng.gen_wait(n_new - 2)  # last token has landed on the host
         eng.gen_end()
-        return out
+        return {"image_embeds": img, "prefill_logits": last, "tokens": [tok0, *out]}
 
     def barrier():
         torch.cuda.synchronize()
@@ -320,8 +350,9 @@ def run_ours(args):
         start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         start.record(stream)
         dec_ms = []
+        dump = {}
         for _ in range(args.steps):
-            figure(True)
+            dump = figure(True)
             stream.synchronize()
             dec_ms.append(ev[1].elapsed_time(ev[2]))
         stop.record(stream)
@@ -352,7 +383,7 @@ def run_ours(args):
             for _ in range(args.steps):
                 model._img_cache = None      # a new figure every step: ViT + full prefill inside the timed region
                 model._slot_tokens = []
-                api_figure()
+                dump["e2e_sequences"] = api_figure()
             torch.cuda.synchronize()
             e2e_t = time.perf_counter() - t0
             barrier()
@@ -369,10 +400,11 @@ def run_ours(args):
                 reps = 5 if B < 64 else 3
                 v0.record(stream)
                 for _ in range(reps):
-                    eng.vit_encode(pix_b)
+                    tokens, pooled = eng.vit_encode(pix_b)
                 v1.record(stream)
                 stream.synchronize()
                 vit[str(B)] = v0.elapsed_time(v1) / reps / B
+                dump[f"vit_b{B}_pooled"], dump[f"vit_b{B}_tokens_sample"] = pooled, seeded_sample(tokens, 1 << 16)
                 del pix_b
         barrier()
 
@@ -409,7 +441,7 @@ def run_ours(args):
             a0, a1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a0.record(stream)
             for _ in range(10):
-                e7.decode([slots7[0]], [ctx7], tok1)
+                logits7 = e7.decode([slots7[0]], [ctx7], tok1)
             a1.record(stream)
             stream.synchronize()
             b1_ms = a0.elapsed_time(a1) / 10
@@ -439,6 +471,8 @@ def run_ours(args):
             g1.record(stream)
             barrier()
             roll_s = g0.elapsed_time(g1) / 1e3
+            dump["ds7b_b1_decode_logits"] = logits7
+            dump["ds7b_rollout_last_tokens"] = local_out
             launches7 = e7.launch_count - l0
         gathered = gather_results([(g, o[:4]) for g, o in zip(figures, local_out)])   # one gather at the end (examples/eval.py:132)
         t7 = torch.tensor([b1_ms, roll_s, float(len(gathered))], dtype=torch.float64)
@@ -532,6 +566,8 @@ def run_ours(args):
                                               f"{r['new_tokens']} greedy tokens at ctx {P}..{P + r['new_tokens']}, {r['dtype']} weights on {r['cores']} threads "
                                               f"(affinity {r['threads']['affinity']}, cgroup quota {r['threads']['cgroup_quota']}); decode tokens/s between first and last new token"}
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dump)
     if world > 1:
         dist.destroy_process_group()
 

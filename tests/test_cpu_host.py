@@ -228,28 +228,20 @@ def test_mcts_tree_growth_and_failed_rollout_memo(monkeypatch):
 
 
 def test_reference_mcts_module_is_drop_in():
-    """The reference's vendored MCTS (importable offline) drives our generator unchanged."""
-    import importlib.util
-    import os
-    base = "/root/reference/detikzify/mcts"
-    if not os.path.isdir(base):
-        pytest.skip("reference checkout not available on this box")
-    mods = {}
-    for n in ("node", "montecarlo"):
-        spec = importlib.util.spec_from_file_location(f"refmcts_{n}", f"{base}/{n}.py")
-        m = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(m)
-        mods[n] = m
-    ours_node = __import__("detikzify_b200.mcts.node", fromlist=["Node"]).Node
-    ref, mine = mods["node"].Node("s"), ours_node("s")
-    for obj in (ref, mine):
-        child = type(obj)("c")
-        obj.add_child(child)
-        child.update_policy_value(1.0)
-        child.update_win_value(0.5)
-    assert ref.visits == mine.visits == 1 and ref.win_value == mine.win_value == 0.5
-    assert ref.children[0].get_score(ref) == pytest.approx(mine.children[0].get_score(mine))
-    assert set(vars(ref)) <= set(vars(mine))
+    """Our MCTS node updates and scores like the reference's vendored MCTS (recorded from it by
+    tests/golden/make_reference_dropin_golden.py) and carries every attribute the reference's node has."""
+    import json
+    from pathlib import Path
+    from detikzify_b200.mcts.node import Node
+    ref = json.loads((Path(__file__).resolve().parent / "golden" / "reference_dropin.json").read_text())["mcts_node"]
+    mine = Node("s")
+    child = Node("c")
+    mine.add_child(child)
+    child.update_policy_value(1.0)
+    child.update_win_value(0.5)
+    assert ref["visits"] == mine.visits == 1 and ref["win_value"] == mine.win_value == 0.5
+    assert mine.children[0].get_score(mine) == pytest.approx(ref["child_score"])
+    assert set(ref["attributes"]) <= set(vars(mine))
 
 
 def test_dyn_minmax_norm():

@@ -1,138 +1,39 @@
 """
-Drop-in boundary (SURVEY.md §8b): the REFERENCE's own inference driver — detikzify/infer/generate.py (DetikzifyGenerator,
-DetikzifyPipeline, WideNode, rollout streaming), detikzify/mcts/*, detikzify/util/{functools,generation}.py, loaded from
-/root/reference and executed unmodified — runs on top of the objects ``detikzify_b200`` returns (model with ``generate``,
-processor, tokenizer), with a scripted engine standing in for the GPU. This is the claim "only the ``load`` import changes".
+Drop-in boundary (SURVEY.md §8b), checked against recordings of the original project: its own inference driver
+(detikzify/infer/generate.py: DetikzifyGenerator, DetikzifyPipeline, WideNode, rollout streaming), its vendored MCTS, its
+SelfSim reward (evaluate/imagesim.py) and its v1 image processor were run on the objects ``detikzify_b200`` returns (model
+with ``generate``, processor, tokenizer), with the scripted engine standing in for the GPU, by
+``tests/golden/make_reference_dropin_golden.py``. What they did — the engine calls and generation kwargs of a sample, the
+programs, scores and tree sizes of MCTS runs, the SelfSim values, the pixels they computed — is stored in
+``tests/golden/reference_dropin.*``.
+Here our own driver, MCTS, SelfSim and processor run on the same objects and must do the same.
 
-Stubbed because they are absent offline and outside the path: torchmetrics (base class only), the TeX toolchain
-(``infer/tikz.py``: pdf2image / pdfCropMargins / pymupdf → a TikzDocument that "compiles" everything), ``util/image.py``
-(pymupdf, requests → two small PIL helpers), ``model/adapter`` (``has_adapter`` → False), POT's ``emd2`` (v1 models pool
-with "cos"). The reference's ``evaluate/imagesim.py`` (SelfSim reward) is loaded for real on a minimal ``torchmetrics.Metric``.
-Skipped on boxes without the reference checkout (the GPU box).
+The recordings were taken with the TeX toolchain stubbed (every program "compiles" into a white 32x32 page); our
+``TikzDocument`` gets the same stand-in renderer here.
 """
-import importlib.util
-import os
-import sys
-import types
+import json
+from pathlib import Path
 
+import numpy as np
 import pytest
 import torch
 from PIL import Image, ImageDraw
 
 from scripted_engine import ScriptedEngine
 
-REF = "/root/reference/detikzify"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not available on this box")
+GOLDEN = Path(__file__).resolve().parent / "golden"
 
 
-def _load(name, path):
-    spec = importlib.util.spec_from_file_location(name, path)
-    mod = importlib.util.module_from_spec(spec)
-    sys.modules[name] = mod
-    spec.loader.exec_module(mod)
-    return mod
+@pytest.fixture(scope="module")
+def gold():
+    return json.loads((GOLDEN / "reference_dropin.json").read_text()), np.load(GOLDEN / "reference_dropin.npz")
 
 
 @pytest.fixture()
-def reference_infer():
-    saved = {k: v for k, v in sys.modules.items() if k.split(".")[0] in ("torchmetrics", "ot", "detikzify")}
-    for k in list(saved):
-        del sys.modules[k]
-    try:
-        tm = types.ModuleType("torchmetrics")
-        tm.Metric = type("Metric", (), {})
-        sys.modules["torchmetrics"] = tm
-        for pkg in ("detikzify", "detikzify.infer", "detikzify.mcts", "detikzify.util", "detikzify.model", "detikzify.evaluate"):
-            m = types.ModuleType(pkg)
-            m.__path__ = []
-            sys.modules[pkg] = m
-        # real reference modules
-        _load("detikzify.mcts.node", f"{REF}/mcts/node.py")
-        _load("detikzify.mcts.montecarlo", f"{REF}/mcts/montecarlo.py")
-        fn = _load("detikzify.util.functools", f"{REF}/util/functools.py")
-        gn = _load("detikzify.util.generation", f"{REF}/util/generation.py")
-        util = sys.modules["detikzify.util"]
-        for mod in (fn, gn):
-            for k, v in vars(mod).items():
-                if not k.startswith("_"):
-                    setattr(util, k, v)
-        util.load = lambda image: image.convert("RGB") if isinstance(image, Image.Image) else Image.open(image).convert("RGB")
-
-        def expand(image, size, do_trim=False):
-            canvas = Image.new("RGB", (size, size), "white")
-            canvas.paste(image, ((size - image.width) // 2, (size - image.height) // 2))
-            return canvas
-        util.expand = expand
-        # stubs for what is absent offline / outside the path
-        adapter = types.ModuleType("detikzify.model.adapter")
-        adapter.has_adapter = lambda model: False
-        sys.modules[adapter.__name__] = adapter
-        adapter.AdapterProcessor = type("AdapterProcessor", (), {})
-        adapter.CrossAttentionAdapterMixin = type("CrossAttentionAdapterMixin", (), {})
-        _load("detikzify.util.torch", f"{REF}/util/torch.py")
-        util.infer_device = sys.modules["detikzify.util.torch"].infer_device
-        # torchmetrics.Metric: the slice of its protocol the reference's ImageSim relies on (states, reset, device/dtype)
-        class Metric(torch.nn.Module):
-            def __init__(self, **kwargs):
-                super().__init__()
-                self._defaults, self._dtype = {}, torch.float32
-
-            def add_state(self, name, default, dist_reduce_fx=None):
-                self._defaults[name] = default
-                setattr(self, name, default.clone())
-
-            def reset(self):
-                for k, v in self._defaults.items():
-                    setattr(self, k, v.clone())
-
-            def set_dtype(self, dtype):
-                self._dtype = dtype
-                return self
-
-            device = property(lambda self: self._device)
-            dtype = property(lambda self: self._dtype)
-        tm.Metric = Metric
-        tmf = types.ModuleType("torchmetrics.functional")
-        tmf.pairwise_cosine_similarity = lambda a, b: torch.nn.functional.normalize(a, dim=-1) @ torch.nn.functional.normalize(b, dim=-1).T
-        sys.modules["torchmetrics.functional"] = tmf
-        ot, otlp = types.ModuleType("ot"), types.ModuleType("ot.lp")
-        def emd2(M, a, b):   # POT's ot.lp.emd2 (absent offline) restated: the transport LP, empty marginals = uniform
-            import numpy as np
-            from scipy.optimize import linprog
-            M = np.asarray(M, dtype=np.float64)
-            n, m = M.shape
-            a = np.full(n, 1.0 / n) if len(a) == 0 else np.asarray(a, dtype=np.float64)
-            b = np.full(m, 1.0 / m) if len(b) == 0 else np.asarray(b, dtype=np.float64)
-            A_eq = np.zeros((n + m, n * m))
-            for i in range(n):
-                A_eq[i, i * m:(i + 1) * m] = 1.0
-            for j in range(m):
-                A_eq[n + j, j::m] = 1.0
-            res = linprog(M.reshape(-1), A_eq=A_eq, b_eq=np.concatenate([a, b]), bounds=(0, None), method="highs")
-            assert res.status == 0, res.message
-            return float(res.fun)
-        otlp.emd2 = emd2
-        sys.modules["ot"], sys.modules["ot.lp"] = ot, otlp
-        _load("detikzify.evaluate.imagesim", f"{REF}/evaluate/imagesim.py")
-        tikz = types.ModuleType("detikzify.infer.tikz")
-
-        class TikzDocument:
-            """Stand-in for the TeX toolchain: every program 'compiles'."""
-            def __init__(self, code, timeout=None):
-                self.code, self.timeout = code, timeout
-            is_rasterizable = True
-            compiled_with_errors = False
-            errors = {}
-
-            def rasterize(self):
-                return Image.new("RGB", (32, 32), "white")
-        tikz.TikzDocument = TikzDocument
-        sys.modules[tikz.__name__] = tikz
-        yield _load("detikzify.infer.generate", f"{REF}/infer/generate.py")
-    finally:
-        for k in [k for k in sys.modules if k.split(".")[0] in ("torchmetrics", "ot", "detikzify")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
+def compiles(monkeypatch):
+    """The stand-in TeX toolchain of the recordings: every program compiles into a white 32x32 page."""
+    from detikzify_b200.infer import TikzDocument
+    monkeypatch.setattr(TikzDocument, "backend", staticmethod(lambda code: Image.new("RGB", (32, 32), "white")))
 
 
 def _ours(eos_at=40):
@@ -151,106 +52,122 @@ def _figure(size=90):
     return im
 
 
-def test_reference_pipeline_sample_runs_on_our_model(reference_infer):
+def _other():
+    im = Image.new("RGB", (80, 80), "white")
+    ImageDraw.Draw(im).ellipse((10, 10, 60, 70), outline="black", width=4)
+    return im
+
+
+def _preprocess_inputs():
+    rng = np.random.default_rng(3)
+    return [_figure(90), _figure(384).resize((384, 384)), Image.fromarray(rng.integers(0, 255, (200, 311, 3), dtype=np.uint8))]
+
+
+# the recorded form of engine calls, documents and sampler arguments (shared with the script that records the original project)
+def calls_json(calls):
+    return json.loads(json.dumps(calls))
+
+
+def doc_json(doc):
+    return {"code": doc.code, "compiled_with_errors": bool(doc.compiled_with_errors), "rasterizable": bool(doc.is_rasterizable)}
+
+
+def sampling_json(kw):
+    """The sampler arguments generate() was given; the RNG seed is drawn per call and is left out."""
+    return {k: v for k, v in kw.items() if k != "seed"}
+
+
+def test_reference_pipeline_sample_runs_on_our_model(gold, compiles):
+    from detikzify_b200.infer import DetikzifyPipeline
+    ref = gold[0]["sample"]
     model, proc, eng = _ours(eos_at=30)
-    pipe = reference_infer.DetikzifyPipeline(model=model, processor=proc, metric="fast")
+    pipe = DetikzifyPipeline(model=model, processor=proc, metric="fast")
+    assert {k: pipe.gen_kwargs.get(k) for k in ref["gen_kwargs"]} == ref["gen_kwargs"]
     assert pipe.gen_kwargs["max_length"] == proc.tokenizer.model_max_length and pipe.gen_kwargs["do_sample"] is True
     doc = pipe.sample(image=_figure())
-    assert isinstance(doc.code, str) and len(doc.code) > 0
-    # the reference passed its own generation kwargs straight into our generate() (infer/generate.py:218-227)
+    assert doc_json(doc) == ref["doc"] and len(doc.code) > 0
+    # the same generation kwargs reach generate() (reference infer/generate.py:218-227), through the same engine calls
     kw = eng.last_sampling
+    assert sampling_json(kw) == ref["sampling"]
     assert kw["bad_token"] == model.config.image_token_id and kw["begin_suppress_token"] == model.config.text_config.eos_token_id
     assert kw["do_sample"] and abs(kw["temperature"] - 0.8) < 1e-6 and abs(kw["top_p"] - 0.95) < 1e-6
+    assert calls_json(eng.calls) == ref["calls"]
 
 
-def test_reference_mcts_simulate_runs_on_our_model(reference_infer):
+def test_reference_mcts_simulate_runs_on_our_model(gold, compiles):
+    from detikzify_b200.infer import DetikzifyPipeline
+    ref = gold[0]["simulate_fast"]
     model, proc, eng = _ours(eos_at=36)
-    pipe = reference_infer.DetikzifyPipeline(model=model, processor=proc, metric="fast")
+    pipe = DetikzifyPipeline(model=model, processor=proc, metric="fast")
     results = list(pipe.simulate(image=_figure(), expansions=4))
-    assert len(results) == 4
-    for score, doc in results:
-        assert score == 1 and isinstance(doc.code, str)          # scorable - compiled_with_errors with the stub compiler
-    # rollouts went through the reference's ThreadPool + TokenStreamer + stopping-criteria path and our streaming contract
+    assert len(results) == 4 and all(score == 1 for score, _ in results)   # scorable - compiled_with_errors
+    # later expansions start wherever the tree search (random among equal scores) goes; the first one is from the root
+    assert [s for s, _ in results] == ref["scores"] and doc_json(results[0][1]) == ref["first_doc"]
+    # rollouts went through the TokenStreamer + stopping-criteria path and our streaming contract
     assert sum(1 for c in eng.calls if c[0] == "gen_begin") >= 4
 
 
-def test_reference_generator_abort_and_tree(reference_infer):
+def test_reference_generator_abort_and_tree(gold, compiles):
+    from detikzify_b200.infer.pipeline import DetikzifyGenerator
+    ref = gold[0]["generator_tree"]
     model, proc, eng = _ours(eos_at=60)
-    gen = reference_infer.DetikzifyGenerator(model=model, processor=proc, image=_figure(), metric=None,
-                                             max_length=proc.tokenizer.model_max_length, temperature=0.8, top_p=0.95, top_k=0,
-                                             do_sample=True)
+    gen = DetikzifyGenerator(model=model, processor=proc, image=_figure(), metric=None, max_length=proc.tokenizer.model_max_length,
+                             temperature=0.8, top_p=0.95, top_k=0, do_sample=True)
     out = [next(gen.simulate(expansions=1)) for _ in range(2)]
     root = gen.montecarlo.root_node
     assert root.visits >= 2 and root.children and root.children[0].is_widen_node
     assert all(score == 1 for score, _ in out)
-    # newline bookkeeping of the reference works with our tokenizer (vocab / decode protocol)
-    assert gen.newlineinfo and all(v.num_lines >= 1 for v in gen.newlineinfo.values())
+    assert [s for s, _ in out] == ref["scores"] and doc_json(out[0][1]) == ref["first_doc"]
+    assert root.visits == ref["root_visits"] and root.children[0].is_widen_node == ref["first_child_widen"]
+    # newline bookkeeping works with our tokenizer (vocab / decode protocol) as the reference's did
+    assert gen.newlineinfo and {str(k): [v.num_lines, v.trailing] for k, v in sorted(gen.newlineinfo.items())} == ref["newlineinfo"]
 
 
-def test_reference_selfsim_metric_runs_on_our_vision_model(reference_infer):
-    """metric="model": the reference's ImageSim.from_detikzify wraps OUR model.model.vision_model / image processor and
-    computes the SelfSim reward from pooler_output (evaluate/imagesim.py:60-125); MCTS then min-max-normalises it."""
+def test_reference_selfsim_metric_runs_on_our_vision_model(gold, compiles):
+    """metric="model": the SelfSim reward wraps OUR model.model.vision_model / image processor and is computed from
+    pooler_output (reference evaluate/imagesim.py:60-125); MCTS then min-max-normalises it."""
+    from detikzify_b200.infer import DetikzifyPipeline
+    ref = gold[0]["simulate_selfsim"]
     model, proc, eng = _ours(eos_at=36)
-    pipe = reference_infer.DetikzifyPipeline(model=model, processor=proc, metric="model")
-    assert type(pipe.metric).__name__ == "ImageSim" and pipe.metric.mode == "cos"
+    pipe = DetikzifyPipeline(model=model, processor=proc, metric="model")
+    assert type(pipe.metric).__name__ == "ImageSim" and pipe.metric.mode == ref["mode"] == "cos"
     pipe.metric.update(img1=_figure(), img2=_figure())
-    assert pipe.metric.compute() == pytest.approx(1.0)            # identical figures -> cosine 1
+    assert pipe.metric.compute() == pytest.approx(ref["same_figure"]) == pytest.approx(1.0)   # identical figures -> cosine 1
     pipe.metric.reset()
     results = list(pipe.simulate(image=_figure(), expansions=3))
     assert len(results) == 3 and all(-1.0 <= score <= 1.0 + 1e-9 for score, _ in results)
+    assert len(ref["scores"]) == 3 and doc_json(results[0][1]) == ref["first_doc"]
     assert any(c[0] == "vit_encode" for c in eng.calls)
 
 
-def test_reference_emd_selfsim_agrees_with_ours(reference_infer):
-    """The v2 default reward: the reference's own ImageSim in "emd" mode (evaluate/imagesim.py:105-107,121-123; POT's emd2
+def test_reference_emd_selfsim_agrees_with_ours(gold):
+    """The v2 default reward: the reference's ImageSim in "emd" mode (evaluate/imagesim.py:105-107,121-123; POT's emd2
     restated as the transport LP) and ours (assignment solver) on the same vision model object and image processor."""
-    from PIL import ImageDraw
     from detikzify_b200.evaluate.imagesim import ImageSim as Ours
-    RefImageSim = sys.modules["detikzify.evaluate.imagesim"].ImageSim
+    ref, arrays = gold[0]["emd"], gold[1]
     model, proc, eng = _ours(eos_at=36)
-    ref = RefImageSim.from_detikzify(model, proc, mode="emd")
     ours = Ours.from_detikzify(model, proc, mode="emd")
-    other = Image.new("RGB", (80, 80), "white")
-    ImageDraw.Draw(other).ellipse((10, 10, 60, 70), outline="black", width=4)
-    # the reference object feeds bf16 pixels (its .to(device, dtype)), ours fp32: compare the solvers on the SAME patch tokens ...
-    f1, f2 = ref.get_vision_features(_figure()), ref.get_vision_features(other)
-    a = ref.get_similarity(_figure(), other)
+    # the reference object fed bf16 pixels (its .to(device, dtype)), ours fp32: compare the solvers on the SAME patch tokens ...
+    f1, f2 = torch.from_numpy(arrays["emd_f1"]), torch.from_numpy(arrays["emd_f2"])
+    a = ref["similarity"]
     assert f1.ndim == 2 and a == pytest.approx(Ours._emd_similarity(f1, f2), abs=1e-9) and -1.0 < a < 1.0
     # ... and the two end-to-end paths within the bf16 rounding of the inputs
-    assert a == pytest.approx(ours.get_similarity(_figure(), other), abs=5e-2)
-    assert ref.get_similarity(_figure(), _figure()) == pytest.approx(1.0, abs=1e-9)
+    assert a == pytest.approx(ours.get_similarity(_figure(), _other()), abs=5e-2)
+    assert ref["same_figure"] == pytest.approx(1.0, abs=1e-9)
+    assert ours.get_similarity(_figure(), _figure()) == pytest.approx(1.0, abs=1e-9)
 
 
-def test_image_processor_matches_reference_preprocess():
+def test_image_processor_matches_reference_preprocess(gold):
     """§8 row a1: our host-side DetikzifyImageProcessor against the reference's own class
-    (detikzify/model/v1/processing_detikzify.py:162-253, loaded from /root/reference; only ``timm.data`` / ``timm.models``,
-    which its ``from_pretrained`` would consult for the SigLIP data config, are stubbed). The instance is built from the
-    dict ``from_pretrained`` assembles (:104-117) with timm's published config of vit_so400m_patch14_siglip_384:
-    input 3x384x384, mean = std = 0.5, bicubic."""
-    import numpy as np
-    saved = {k: v for k, v in sys.modules.items() if k.split(".")[0] == "timm"}
-    try:
-        timm = types.ModuleType("timm"); timm.__path__ = []
-        data, models = types.ModuleType("timm.data"), types.ModuleType("timm.models")
-        cfg = {"input_size": [3, 384, 384], "mean": (0.5, 0.5, 0.5), "std": (0.5, 0.5, 0.5), "crop_mode": "center"}
-        models.resolve_pretrained_cfg = lambda variant: types.SimpleNamespace(to_dict=lambda: dict(cfg))
-        data.resolve_data_config = lambda d: dict(d)
-        sys.modules.update({"timm": timm, "timm.data": data, "timm.models": models})
-        ref_mod = _load("ref_processing_detikzify", f"{REF}/model/v1/processing_detikzify.py")
-        ref = ref_mod.DetikzifyImageProcessor.from_pretrained("vit_so400m_patch14_siglip_384.webli")
-    finally:
-        for k in [k for k in sys.modules if k.split(".")[0] == "timm"]:
-            del sys.modules[k]
-        sys.modules.update(saved)
-        sys.modules.pop("ref_processing_detikzify", None)
+    (detikzify/model/v1/processing_detikzify.py:162-253), built from the dict its ``from_pretrained`` assembles (:104-117)
+    with timm's published config of vit_so400m_patch14_siglip_384: input 3x384x384, mean = std = 0.5, bicubic."""
     from detikzify_b200.model.processing import DetikzifyImageProcessor
+    ref, arrays = gold[0]["image_processor"], gold[1]
     ours = DetikzifyImageProcessor(size=384)
-    assert ref.size == ours.size and list(ref.image_mean) == ours.image_mean and list(ref.image_std) == ours.image_std
-    assert int(ref.resample) == ours.resample == 3 and abs(ref.rescale_factor - ours.rescale_factor) < 1e-12
-    rng = np.random.default_rng(3)
-    images = [_figure(90), _figure(384).resize((384, 384)), Image.fromarray(rng.integers(0, 255, (200, 311, 3), dtype=np.uint8))]
-    for im in images:
-        a = ref(images=im, return_tensors="pt")["pixel_values"]
+    assert ref["size"] == ours.size and ref["image_mean"] == ours.image_mean and ref["image_std"] == ours.image_std
+    assert ref["resample"] == ours.resample == 3 and abs(ref["rescale_factor"] - ours.rescale_factor) < 1e-12
+    for i, im in enumerate(_preprocess_inputs()):
+        a = (torch.from_numpy(arrays[f"pixels_{i}"]).double() / 255 - 0.5) / 0.5
         b = ours(im, return_tensors="pt")["pixel_values"]
         assert a.shape == b.shape == (1, 3, 384, 384) and b.dtype == torch.float32
-        assert (a.float() - b).abs().max().item() < 1e-6
+        assert (a - b.double()).abs().max().item() < 1e-6
