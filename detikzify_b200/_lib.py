@@ -73,6 +73,10 @@ SYMBOLS = {
     "dtk_dbg_gemm": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P]),
     "dtk_dbg_flash_attn": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_float, _P]),
+    "dtk_dbg_flash_attn_ex": (C.c_int, [_P, _P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                        C.c_int, C.c_int, C.c_int, C.c_float, _P]),
+    "dtk_dbg_decode_attn": (C.c_int, [_P, _P, C.c_int, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                      C.c_float, _P, _P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, _P]),
     "dtk_dbg_attn_tc": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_float, _P]),
     "dtk_dbg_gemv": (C.c_int, [_P, _P, _P, C.c_float, C.c_int, C.c_int, C.c_int, _P, _P]),
 }

@@ -1335,6 +1335,82 @@ int dtk_dbg_flash_attn(const void* q, const void* k, const void* v, void* o, int
   return launch_flash_attn(a, (cudaStream_t)stream, nullptr) == cudaSuccess ? DTK_OK : DTK_ERR_CUDA;
 }
 
+int dtk_dbg_flash_attn_ex(const void* q, const void* k, const void* v, const void* k2, const void* v2, void* o, int B,
+                          int heads, int kv_heads, int Tq, int Tk, int head_dim, int causal, int q_pos0, int split_row,
+                          float scale, void* stream) {
+  if (!q || !k || !v || !o || B <= 0 || heads <= 0 || kv_heads <= 0 || heads % kv_heads || Tq <= 0 || Tk <= 0)
+    return DTK_ERR_INVALID;
+  if ((head_dim != 72 && head_dim != 128) || q_pos0 < 0 || split_row < 0 || split_row > Tk) return DTK_ERR_INVALID;
+  if (split_row > 0 && (!k2 || !v2)) return DTK_ERR_INVALID;
+  AttnArgs a{};
+  a.q = (const bf16*)q; a.k = (const bf16*)k; a.v = (const bf16*)v; a.o = (bf16*)o;
+  a.k2 = (const bf16*)k2; a.v2 = (const bf16*)v2; a.split_row = split_row;
+  const int64_t rs = (int64_t)heads * head_dim, krs = (int64_t)kv_heads * head_dim;
+  a.q_bs = (int64_t)Tq * rs; a.q_hs = head_dim; a.q_rs = rs;
+  a.k_bs = (int64_t)Tk * krs; a.k_hs = head_dim; a.k_rs = krs;
+  a.v_bs = (int64_t)Tk * krs; a.v_hs = head_dim; a.v_rs = krs;
+  a.o_bs = (int64_t)Tq * rs; a.o_hs = head_dim; a.o_rs = rs;
+  a.B = B; a.heads = heads; a.kv_group = heads / kv_heads; a.Tq = Tq; a.Tk = Tk; a.q_pos0 = q_pos0; a.causal = causal;
+  a.head_dim = head_dim; a.scale = scale;
+  return launch_flash_attn(a, (cudaStream_t)stream, nullptr) == cudaSuccess ? DTK_OK : DTK_ERR_CUDA;
+}
+
+int dtk_dbg_decode_attn(const float* q, const void* kv, int nslots, const int* slots, const int* pos,
+                        const int* share_slot, const int* share_len, int B, int heads, int kv_heads, int max_len,
+                        int nsplit, float scale, float* part_o, float* part_ml, unsigned int* counters, float* out,
+                        void* out_bf16, const void* q_bf16, int prefix_slot, int prefix_len, int part_tiles,
+                        void* stream) {
+  if (!q || !kv || !slots || !pos || !part_o || !part_ml || !counters || !out) return DTK_ERR_INVALID;
+  if (B <= 0 || B > 64 || heads <= 0 || kv_heads <= 0 || heads % kv_heads || max_len <= 0 || nslots <= 0)
+    return DTK_ERR_INVALID;
+  if (nsplit < 1 || nsplit > 16 || prefix_len < 0 || prefix_len > max_len) return DTK_ERR_INVALID;
+  int csplit = 0;
+  if (prefix_len > 0) {   // the engine's shared-prefix ("cascade") pass: launch_flash_attn in partial mode, then the merge
+    if (!q_bf16 || part_tiles <= 0 || prefix_slot < 0 || prefix_slot >= nslots) return DTK_ERR_INVALID;
+    csplit = ((prefix_len + 63) / 64 + part_tiles - 1) / part_tiles;
+    if (nsplit + csplit > 16) return DTK_ERR_INVALID;   // partial buffers hold 16 slots per (row, head)
+  }
+  // the per-row state lives on the device: check it on the host so that no launch indexes outside the KV buffer
+  std::vector<int> h_slots(B), h_pos(B), h_sslot(B, 0), h_slen(B, 0);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (cudaStreamSynchronize(s) != cudaSuccess) return DTK_ERR_CUDA;
+  bool ok = cudaMemcpy(h_slots.data(), slots, B * sizeof(int), cudaMemcpyDeviceToHost) == cudaSuccess &&
+            cudaMemcpy(h_pos.data(), pos, B * sizeof(int), cudaMemcpyDeviceToHost) == cudaSuccess;
+  if (ok && share_len) {
+    if (!share_slot) return DTK_ERR_INVALID;
+    ok = cudaMemcpy(h_sslot.data(), share_slot, B * sizeof(int), cudaMemcpyDeviceToHost) == cudaSuccess &&
+         cudaMemcpy(h_slen.data(), share_len, B * sizeof(int), cudaMemcpyDeviceToHost) == cudaSuccess;
+  }
+  if (!ok) return DTK_ERR_CUDA;
+  for (int b = 0; b < B; ++b) {
+    if (h_slots[b] < 0 || h_slots[b] >= nslots || h_pos[b] < prefix_len || h_pos[b] >= max_len) return DTK_ERR_INVALID;
+    if (h_slen[b] < 0 || h_slen[b] > max_len) return DTK_ERR_INVALID;
+    if (h_slen[b] > 0 && (h_sslot[b] < 0 || h_sslot[b] >= nslots)) return DTK_ERR_INVALID;
+  }
+  // one layer of the engine's slot-major cache: [slot][K | V][kv_head][max_len][128]
+  const int64_t v_off = (int64_t)kv_heads * max_len * 128;
+  const bf16* kvb = (const bf16*)kv;
+  if (prefix_len > 0) {
+    AttnArgs f{};
+    f.q = (const bf16*)q_bf16; f.k = kvb + prefix_slot * 2 * v_off; f.v = f.k + v_off;
+    f.q_bs = 0; f.q_hs = 128; f.q_rs = (int64_t)heads * 128;
+    f.k_bs = 0; f.k_hs = (int64_t)max_len * 128; f.k_rs = 128;
+    f.v_bs = 0; f.v_hs = (int64_t)max_len * 128; f.v_rs = 128;
+    f.B = 1; f.heads = heads; f.kv_group = heads / kv_heads; f.Tq = B; f.Tk = prefix_len; f.q_pos0 = 0;
+    f.causal = 0; f.head_dim = 128; f.scale = scale;
+    f.part_o = part_o; f.part_ml = part_ml; f.part_np = nsplit + csplit; f.part_idx0 = nsplit; f.part_tiles = part_tiles;
+    if (launch_flash_attn(f, s, nullptr) != cudaSuccess) return DTK_ERR_CUDA;
+  }
+  DecodeAttnArgs a{};
+  a.q = q; a.q_stride = (int64_t)heads * 128; a.kv_base = kvb; a.kv_slot_stride = 2 * v_off; a.kv_v_offset = v_off;
+  a.slots = slots; a.pos = pos; a.share_slot = share_slot; a.share_len = share_len;
+  a.B = B; a.heads = heads; a.kv_group = heads / kv_heads; a.max_len = max_len; a.nsplit = nsplit; a.scale = scale;
+  a.part_o = part_o; a.part_ml = part_ml; a.counters = counters;
+  a.out = out; a.out_stride = (int64_t)heads * 128; a.out_bf16 = (bf16*)out_bf16;
+  if (prefix_len > 0) { a.key_begin = prefix_len; a.np = nsplit + csplit; }
+  return launch_decode_attn(a, s, nullptr) == cudaSuccess ? DTK_OK : DTK_ERR_CUDA;
+}
+
 int dtk_dbg_attn_tc(const void* qkv, void* vt_scratch, void* o, int B, int heads, int N, float scale, void* stream) {
   if (!qkv || !vt_scratch || !o || B <= 0 || heads <= 0 || N <= 0) return DTK_ERR_INVALID;
   if (!attn_tc_supported()) return DTK_ERR_UNSUPPORTED;

@@ -215,6 +215,27 @@ DTK_API int dtk_dbg_gemm(const void* A_bf16, const void* W_bf16, const void* bia
 DTK_API int dtk_dbg_flash_attn(const void* q, const void* k, const void* v, void* o, int B,
                                int heads, int Tq, int Tk, int head_dim, int causal, int q_pos0,
                                float scale, void* stream);
+/* dtk_dbg_flash_attn with grouped KV heads and a borrowed prefix: q, o bf16 [B, Tq, heads, head_dim]; k, v, k2, v2 bf16
+ * [B, Tk, kv_heads, head_dim] (query head h reads KV head h / (heads / kv_heads)); key rows below split_row are read from
+ * k2 / v2, the others from k / v (split_row = 0: k2 / v2 unused, may be NULL). Returns DTK_ERR_INVALID on bad arguments. */
+DTK_API int dtk_dbg_flash_attn_ex(const void* q, const void* k, const void* v, const void* k2, const void* v2, void* o,
+                                  int B, int heads, int kv_heads, int Tq, int Tk, int head_dim, int causal, int q_pos0,
+                                  int split_row, float scale, void* stream);
+/* split-KV single-query decode attention over one layer of a caller-owned slot cache kv bf16
+ * [nslots][K | V][kv_heads][max_len][128]. q fp32 [B, heads*128]; slots, pos, share_slot, share_len device int32 [B]
+ * (row b attends keys [0, pos[b]]; keys below share_len[b] come from slot share_slot[b]; share_len may be NULL);
+ * part_o fp32 [B, heads, 16, 128], part_ml fp32 [B, heads, 16, 2] scratch; counters uint32 [B*heads], zero on entry and
+ * zero again on return; out fp32 [B, heads*128], out_bf16 (may be NULL) the same in bf16. nsplit key ranges per (row, head).
+ * prefix_len > 0 runs the shared-prefix pass of batched decode first: keys [0, prefix_len) of slot prefix_slot are reduced
+ * for all rows by the tensor-core kernel (q_bf16 bf16 [B, heads*128], part_tiles 64-key tiles per CTA) into partial slots
+ * [nsplit, nsplit + csplit), csplit = ceil(ceil(prefix_len / 64) / part_tiles), and the per-row pass covers
+ * [prefix_len, pos[b]]. B <= 64, nsplit + csplit <= 16, pos[b] >= prefix_len; row state is checked on the host (the call
+ * synchronises `stream`). Returns DTK_ERR_INVALID on bad arguments. */
+DTK_API int dtk_dbg_decode_attn(const float* q, const void* kv, int nslots, const int* slots, const int* pos,
+                                const int* share_slot, const int* share_len, int B, int heads, int kv_heads, int max_len,
+                                int nsplit, float scale, float* part_o, float* part_ml, unsigned int* counters,
+                                float* out, void* out_bf16, const void* q_bf16, int prefix_slot, int prefix_len,
+                                int part_tiles, void* stream);
 /* ViT attention on tcgen05: qkv bf16 [B*N, 3*heads*72] (q | k | v column blocks), vt_scratch bf16 [B*heads*80, ceil(N/128)*128],
  * o bf16 [B*N, heads*72]; non-causal, head_dim 72 */
 DTK_API int dtk_dbg_attn_tc(const void* qkv, void* vt_scratch, void* o, int B, int heads, int N, float scale, void* stream);
